@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one rank per GPU)
   python bench.py --impl reference --steps K --warmup W    # the reference algorithm on the host cores
+  python bench.py ... --dump-outputs DIR                   # also write what the last timed step computed (DIR/*.npy)
 
 A "step" is ONE Levenberg-Marquardt iteration of the reference's loop (solver/bal_bundle_adjustment.cpp:291-521):
 [compute_error + linearize at a new linearization point] + solve(lambda) + apply + compute_error + accept/reject.
@@ -394,6 +395,26 @@ def trajectory_fields(st) -> dict:
             "final_cost": next((r.get("cost") for r in reversed(st.log) if r.get("cost") is not None and r.get("cost") == r.get("cost")), None)}
 
 
+LAST_STEP_FIELDS = ("lambda", "cost", "l_diff", "relative_decrease", "cg_iterations", "accepted", "terminated")
+DUMP_BUDGET_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, lin, last):
+    """What the timed LM loop hands its caller after its last step, as DIR/<name>.npy: the camera and landmark state (the
+    landmarks of this rank's shard) in the solver's scalar type, and that step's record (LAST_STEP_FIELDS, float64).
+    Landmarks that would exceed DUMP_BUDGET_BYTES are cut to a fixed, seeded sample of rows, the same rows in every run."""
+    lin.download_state()
+    bp, stats = lin.bal_problem, lin.stats()
+    lms = bp.lms[stats["landmark_begin"]:stats["landmark_end"]]
+    room = (DUMP_BUDGET_BYTES - bp.cams.nbytes - 4096) // (3 * bp.lms.itemsize)
+    if len(lms) > room:
+        lms = lms[np.sort(np.random.default_rng(0).choice(len(lms), room, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("cameras", bp.cams), ("landmarks", lms),
+                    ("last_step", np.array([last[k] for k in LAST_STEP_FIELDS], dtype=np.float64))):
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def bench_reference(args):
     """the reference's algorithm (CPU restatement, oracle/) on the host cores; rank 0 only"""
     rank = int(os.environ.get("RANK", "0"))
@@ -505,8 +526,10 @@ def bench_ours(args):
                     step_ms.extend(1e3 * i["device_seconds"] for i in its)
                     for k in PH:
                         phase[k] += tot[k]
-                if term or left > 0:
-                    be.reset()  # a new solve from the initial point
+                if left > 0:
+                    be.reset()  # the solve ended: a new solve from the initial point
+            # a solve that ends with the last step is not reset here: its state is the result of that step, and the
+            # reset belongs to the next solve, which is not timed
 
         run(args.warmup, False)
         be.reset()
@@ -531,6 +554,8 @@ def bench_ours(args):
         sampler.start()
     lin = make_linearizor()
     dev_s, wall_s, st, phase, step_ms, launches = timed_run(lin)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, lin, st.log[-1])
     secs = torch.tensor([dev_s], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(secs, op=dist.ReduceOp.MAX)
@@ -653,7 +678,14 @@ def main():
     ap.add_argument("--cpu-budget-s", type=float, default=150.0, help="reference arm: wall-time budget of the timed steps")
     ap.add_argument("--operator", default="dense", choices=["dense", "implicit"],
                     help="PCG operator form: dense = the reference's Q2-panel product (default, contract kernel); implicit = opt-in")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the state after the last one (cameras, landmarks) and that step's "
+                         f"record (last_step: {', '.join(LAST_STEP_FIELDS)}) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computes (--impl ours)")
     if args.workload is None:
         args.workload = default_workload(args.gpus)
     if args.impl == "reference":

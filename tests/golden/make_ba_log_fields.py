@@ -1,15 +1,18 @@
 #!/usr/bin/env python
 """Extract the field names (in declaration order) of the reference's BaLog structs from
-/root/reference/src/rootba/bal/ba_log.hpp into tests/golden/ba_log_fields.json.
+<rootba checkout>/src/rootba/bal/ba_log.hpp into tests/golden/ba_log_fields.json.
 
-Run in the build container (the reference tree is not available on the GPU box); the JSON is committed.
+    python tests/golden/make_ba_log_fields.py <rootba checkout>
+
+The JSON is committed, so the tests do not need the reference.
 The per-iteration structs become top-level columns of ba_log.json, the others live under "_static"
 (src/rootba/bal/ba_log.cpp:62-150)."""
 import json
 import os
 import re
+import sys
 
-SRC = "/root/reference/src/rootba/bal/ba_log.hpp"
+SRC = os.path.join(sys.argv[1], "src", "rootba", "bal", "ba_log.hpp")
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "ba_log_fields.json")
 
 txt = open(SRC).read()

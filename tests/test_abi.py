@@ -20,14 +20,22 @@ def test_library_exports_every_declared_symbol():
     assert L.rba_abi_version() == 1
 
 
-def test_no_cpu_fallback(tiny_problem):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    bp = rb.BalProblem.from_arrays(tiny_problem)
-    with pytest.raises(rb.RbaError) as e:
-        rb.LinearizorQR.create(bp, rb.SolverOptions())
-    assert e.value.code == -2  # RBA_ERR_NO_DEVICE
+def test_no_cpu_fallback():
+    """run in a child process with every device hidden, so that the check holds on a machine with a GPU too"""
+    import subprocess
+    import sys
+    from conftest import ROOT
+    code = ("import rootba_b200 as rb\n"
+            "from rootba_b200.synthetic import synth_bal\n"
+            "bp = rb.BalProblem.from_arrays(synth_bal(12, 300, 4.1, seed=1))\n"
+            "try:\n"
+            "    rb.LinearizorQR.create(bp, rb.SolverOptions())\n"
+            "except rb.RbaError as e:\n"
+            "    print('code', e.code)\n")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert r.stdout.split() == ["code", "-2"]  # RBA_ERR_NO_DEVICE
 
 
 def test_partition_landmarks(small_problem):
