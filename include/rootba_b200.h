@@ -252,8 +252,10 @@ int32_t rba_lm_step_f64(rba_handle* h, int32_t linearize_first, double lambda, r
 /* The LM loop itself, natively: optimize_lm_ours (solver/bal_bundle_adjustment.cpp:291-521) on top of rba_lm_step, so that
  * consecutive iterations are separated by one host synchronisation and a few scalar operations instead of an interpreter.
  * Starts a NEW solve at the handle's current state (lambda = 1 / initial_trust_region_radius, vee = initial_vee) and runs
- * until the reference's stopping rule fires -- |cost change| <= function_tolerance * cost after a successful step (:174-201),
- * lambda > 1 / min_trust_region_radius (:378-379), max_num_iterations (:291) -- or `max_steps` iterations have been done.
+ * until the reference's stopping rule fires -- after a successful step, |previous logged cost - cost| <= function_tolerance *
+ * cost (:69-72, :174-201), where the previous logged cost is that of the iteration before (the initial cost, a rejected step's
+ * cost, or 0 after a failed solve) and both are in the ERROR / ERROR_VALID sense; lambda > 1 / min_trust_region_radius
+ * (:378-379); max_num_iterations (:291) -- or `max_steps` iterations have been done.
  * Same Scalar arithmetic for lambda / vee / step quality as the reference loop (and as the Python / C++ host mirrors, which
  * stay the tested restatements).  One rba_lm_iteration is written per iteration. */
 typedef struct {

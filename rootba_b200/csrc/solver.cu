@@ -790,13 +790,16 @@ struct Solver : rba_handle {
     return launch_ex(k_pcg_vec<S>, pcg_cluster, VEC_THREADS, 0, pdl && use_pdl, pcg_cluster, D, d_state, lambda, i, mode, (double)opt.eta,
                      (int)opt.min_linear_solver_iterations, is_last, (int)(pdl && use_pdl), c, ar_seq, from_partials ? op_item_ptr : (const int*)nullptr, d_prog);
   }
+  // The hand-over through per-segment sums is taken when a cluster CTA's share of the cameras fits the vector kernel's
+  // register-resident layout: 9 * ceil(nc / cluster) <= VEC_THREADS * VEC_EPT = 1024, i.e. <= 1808 cameras with a 16-CTA
+  // cluster.  Larger camera counts on one GPU (Final-13682) keep the arrival-counter reduction into D.y (pcg_apply), the
+  // combination that was measured at that size.
+  bool pcg_from_partials() const {
+    return opt.nranks == 1 && pcg_partials && 9 * ((nc + pcg_cluster - 1) / pcg_cluster) <= VEC_THREADS * VEC_EPT;
+  }
   // finish one operator application inside PCG (H v for v = p in mode 0/1, x in mode 2) and do the vector step
   int pcg_apply(int i, int mode, int is_last, S lambda) {
-    // The hand-over through per-segment sums is taken when a cluster CTA's share of the cameras fits the vector kernel's
-    // register-resident layout (<= 1820 cameras with a 16-CTA cluster); larger camera counts on one GPU (Final-13682)
-    // keep the arrival-counter reduction below, the combination that was measured at that size.
-    const bool vec_cached = 9 * ((nc + pcg_cluster - 1) / pcg_cluster) <= VEC_THREADS * VEC_EPT;
-    if (opt.nranks == 1 && pcg_partials && vec_cached) {
+    if (pcg_from_partials()) {
       // one GPU: the vector kernel adds the per-segment sums itself (same order as k_cam_reduce_final's last arriver:
       // bit-identical) -- no arrival counters, fences or second pass in the reduction
       int rc = launch_ex(k_cam_reduce<S>, grid_for(n_op_items, 8, 8), 256, 0, use_pdl, 1, (const S*)D.yobs, op_slots, op_items, n_op_items, D.partial,
@@ -896,6 +899,10 @@ struct Solver : rba_handle {
     rc = stop(ev_precond); if (rc) return rc;
     last_lambda = lambda;
     damping_valid = true;
+    // One GPU, operator sums through D.y (Power-SC, or PCG without the per-segment hand-over): k_cam_reduce_final writes y only
+    // for cameras that have observations, so the others must start at 0 -- not at what rba_right_multiply left there
+    // (H x + lambda x).  Every iteration of the solve then leaves them 0.
+    if (opt.nranks == 1 && (power || !pcg_from_partials())) CU(cudaMemsetAsync(D.y, 0, (size_t)9 * nc * sizeof(S), stream));
     if (power) return power_enqueue(inc_out);
     // PCG (ref: cg/conjugate_gradient.hpp:113-298 ; linearizor_base.cpp:81-103)
     rc = start(ev_pcg); if (rc) return rc;
@@ -1067,6 +1074,10 @@ struct Solver : rba_handle {
     S lam = (S)(1.0 / o->initial_trust_region_radius), vee = initial_vee;
     bool new_outer = true, terminated = false;
     rba_residual_info ri{};
+    // cost of the previous log entry in the ERROR / ERROR_VALID sense, which the function tolerance compares against
+    // (:69-72, :174-201): the initial cost, then every logged step's cost -- a rejected step's too -- and 0 after a failed solve
+    const int prev_kind = o->optimized_cost == 0 ? 0 : 1;
+    double prev_logged = 0;
     if (totals) std::memset(totals, 0, sizeof(*totals));
     int it = 0;
     for (; it < max_steps && !terminated; ++it) {
@@ -1078,6 +1089,7 @@ struct Solver : rba_handle {
       if (new_outer) {
         int rc = compute_error(&ri); if (rc) return rc;   // answered from the cache after an accepted step
         if (!ri.is_numerically_valid) { g_err = "did not expect numerical failure during linearization"; return RBA_NUMERICAL_FAILURE; }  // :307-308
+        if (it == 0) prev_logged = cost_of(ri, prev_kind);
         dev += tm.residual_evaluation_time;
         if (totals) totals->residual_evaluation_time += tm.residual_evaluation_time;
         new_outer = false;
@@ -1101,10 +1113,14 @@ struct Solver : rba_handle {
       L2.l_diff = r.l_diff;
       L2.cost = std::numeric_limits<double>::quiet_NaN();
       bool success = false;
+      const double prev = prev_logged;
       if (r.solve_failed) {
         // non-finite increment (:360-399): not applied by the reference; here undone
         rc = restore(); if (rc) return rc;
+        prev_logged = 0;
       } else {
+        const double cur = cost_of(r.cost, prev_kind);
+        prev_logged = cur;
         const S l_diff = (S)r.l_diff;
         const bool ok = std::isfinite((double)l_diff) && r.cost.is_numerically_valid;
         L2.cost = cost_of(r.cost, o->optimized_cost);
@@ -1121,7 +1137,6 @@ struct Solver : rba_handle {
             lam = std::max(min_lambda, lam);
             vee = initial_vee;
             new_outer = true;
-            const double prev = cost_of(ri, o->optimized_cost == 0 ? 0 : 1), cur = cost_of(r.cost, o->optimized_cost == 0 ? 0 : 1);
             terminated = std::fabs(prev - cur) <= o->function_tolerance * cur;  // function_tolerance_reached (:174-201)
           }
         }

@@ -49,6 +49,12 @@ def make_pair(arrays, dtype, **opt_kw):
         so.stage2_form = opt_kw["stage2_form"]      # device-side choice only: the oracle always reads the Q2 panel
     if "max_num_iterations" in opt_kw:
         so.max_num_iterations = okw["max_num_iterations"] = opt_kw["max_num_iterations"]
+    for k in ("min_linear_solver_iterations", "max_linear_solver_iterations", "eta"):  # PCG stopping rule, both sides
+        if k in opt_kw:
+            setattr(so, k, opt_kw[k])
+            okw[k] = opt_kw[k]
+    if "pcg_check_period" in opt_kw:
+        so.pcg_check_period = opt_kw["pcg_check_period"]  # device-side scheduling only
     bp = rb.BalProblem.from_arrays(arrays, dtype)
     lin = rb.LinearizorQR.create(bp, so)
     o = orc.Oracle(arrays, dtype, orc.default_options(num_threads=0, **okw))

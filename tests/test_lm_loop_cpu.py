@@ -173,3 +173,30 @@ def test_cpp_lm_loop_equals_oracle_lm_loop(tmp_path, small_problem, hard_problem
             assert a["cg"] == int(b["cg_iterations"]) and a["rho"] == pytest.approx(b["relative_decrease"], rel=1e-9, abs=1e-12)
     if hard:
         assert not all(a["ok"] for a in got[1:])
+
+
+def test_function_tolerance_compares_with_the_previous_logged_cost():
+    """The stop after a successful step compares its cost with the previous log entry's (bal_bundle_adjustment.cpp:69-72,
+    :174-201), which after rejected steps is the last rejected cost.  Here iterations 1-6 are rejected and 7 is accepted
+    with a cost within 10% of the linearisation point's but 62% away from iteration 6's, so the loop goes on and stops at
+    iteration 10.  Pinned for the oracle and the Python mirror; tests/test_gpu_pcg_paths.py holds rba_lm_run to it."""
+    from rootba_b200.synthetic import synth_bal
+    prob = synth_bal(49, 1800, 4.1, seed=38401, perturb_rot=0.2, perturb_trans=1.0, perturb_lm=2.0)
+    kw = dict(max_num_iterations=20, min_relative_decrease=0.99, function_tolerance=0.1)
+    rows, term = orc.Oracle(prob, np.float64, orc.default_options(num_threads=1, **kw)).optimize()
+    assert [bool(r["step_is_successful"]) for r in rows] == [True] + [False] * 6 + [True, False, False, True]
+    assert term == 1  # CONVERGENCE
+    c = [r["cost"] for r in rows]
+    assert abs(c[0] - c[7]) <= 0.1 * c[7] < abs(c[6] - c[7])  # the linearisation point's cost would have stopped at 7
+    assert abs(c[9] - c[10]) <= 0.1 * c[10]  # the rejected iteration 9's cost stops at 10
+    drv = orc.Oracle(prob, np.float64, orc.default_options(num_threads=1, **kw))
+    bp = rb.BalProblem.from_arrays(prob, np.float64)
+    lin = OracleLinearizor(drv)
+    bp._linearizor = lin
+    summ = rb.bundle_adjust_manual(bp, rb.SolverOptions(**kw), linearizor=lin)
+    its = summ["iterations"]
+    assert summ["termination_type"] == "CONVERGENCE" and len(its) == len(rows)
+    for a, b in zip(its, rows):
+        assert bool(a["step_is_successful"]) == bool(b["step_is_successful"]) and a["cost"]["all"]["error"] == b["cost"]
+        if a["iteration"] > 0:
+            assert a["linear_solver_iterations"] == int(b["cg_iterations"])
